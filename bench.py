@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one JSON line on rank 0)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port) on the host cores
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR # also write the last timed step's outputs to DIR/*.npy
 
 Primary line (`value`, `e2e`, `roofline`): BASELINE.json config 3 — 65 536 particles x 256 landmarks PER GPU (weak scaling:
 global = 65 536 x N), ~12.7 of 256 landmarks observed per step, nth = particles / 1.5.  A "step" = one fastslam_update
@@ -208,6 +209,69 @@ def load_traffic():
         return {"traffic": None}
 
 
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed in its last timed step, as float64 .npy files, so that two builds can be
+# compared output for output on identical (seeded) inputs
+# ------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_MAP_PARTICLES = 256       # landmark maps are n x m x 48 bytes: a fixed, seeded sample of particles is written
+DUMP_ROWS_BYTES = 48 << 20     # larger particle arrays are written as a fixed, seeded sample of rows
+
+
+def seeded_sample(n, k):
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(12345).choice(n, size=k, replace=False))
+
+
+def sample_rows(name, a, out):
+    """a whole when it fits DUMP_ROWS_BYTES, else a fixed, seeded sample of its rows (and `<name>_index`, the rows taken)"""
+    per_row = a.nbytes // max(a.shape[0], 1)
+    idx = seeded_sample(a.shape[0], max(1, DUMP_ROWS_BYTES // max(per_row, 1)))
+    if idx.size == a.shape[0]:
+        out[name] = a
+    else:
+        out[name] = a[idx]
+        out[name + "_index"] = idx
+
+
+def fastslam_outputs(g):
+    """what a caller of fastslam_update holds after the step: every particle's (weight, x, y, yaw), the landmark maps
+    (x, y, c00, c01, c10, c11 per landmark) of a seeded sample of particles, get_best_particle(), and whether it resampled"""
+    import numpy as np
+    out = {}
+    poses, _ = g.state(landmarks=False)
+    sample_rows("particles", poses, out)
+    pick = seeded_sample(g.n_local, DUMP_MAP_PARTICLES)
+    out["landmarks"] = np.stack([g.particle_landmarks(int(i)) for i in pick])
+    out["landmarks_index"] = pick
+    best, best_pose = g.get_best_particle()
+    out["best_index"] = np.array([best])
+    out["best_particle"] = best_pose
+    out["resampled"] = np.array([g.last_gate()])
+    return out
+
+
+def pf_outputs(g):
+    """what a caller of try_step holds after the step: the particles (x, y, yaw, v, weight) and estimate()"""
+    out = {}
+    sample_rows("particles", g.get_particles(), out)
+    out["estimate"] = g.estimate()
+    return out
+
+
+def write_outputs(d, arrays, suffix=""):
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, f"{k}{suffix}.npy"), a)
+
+
 CONFIGS = {   # SURVEY.md §8(d)
     "c3": dict(name="FastSLAM 1.0 (fs1.rs fastslam_update), BASELINE config 3", particles_per_gpu=N_PARTICLES, particles_total=None,
                scenario="c3_scenario", scaling="weak"),
@@ -237,8 +301,9 @@ def make_engine(rr, grp, cfg_key, rank, world, local_rank):
     return cfg, n_global, scenarios, rdist
 
 
-def measure(rr, grp, cfg_key, K, W, rank, world, local_rank, with_e2e, sampler_cb=None):
-    """one configuration: warm-up, K flushed + event-timed steps, K un-flushed steps, (optionally) K end-to-end steps"""
+def measure(rr, grp, cfg_key, K, W, rank, world, local_rank, with_e2e, sampler_cb=None, dump_dir=None):
+    """one configuration: warm-up, K flushed + event-timed steps, K un-flushed steps, (optionally) K end-to-end steps.
+    dump_dir: write the outputs of the last of the K steps `value` is quoted on (each rank its own shard)"""
     from rust_robotics_b200 import dist as rdist, scenarios
     cfg = CONFIGS[cfg_key]
     n_global = cfg["particles_total"] or cfg["particles_per_gpu"] * world
@@ -287,6 +352,8 @@ def measure(rr, grp, cfg_key, K, W, rank, world, local_rank, with_e2e, sampler_c
     # pass A: the K steps `value` is quoted on.  No events inside a step: an event pair around the EKF launch costs ~8 us per step (it
     # breaks the programmatic dependent launch of the kernel behind it), so the kernel is timed on its own pass below.
     first, step_ms, st0, st1 = flushed_pass(False)
+    if dump_dir:
+        write_outputs(dump_dir, fastslam_outputs(g), "" if world == 1 else f"_rank{rank}")
     if os.environ.get("BENCH_VERBOSE") and rank == 0:
         ss = sorted(step_ms)
         sys.stderr.write("step ms: min %.3f  p50 %.3f  p90 %.3f  p99 %.3f  max %.3f  sum %.1f; worst steps %s\n" % (
@@ -361,11 +428,11 @@ def run_ours(args, rank, world, local_rank):
     grp = rdist.TcpGroup()
     K, W = args.steps, args.warmup
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    primary = measure(rr, grp, args.config, K, W, rank, world, local_rank, True)
+    primary = measure(rr, grp, args.config, K, W, rank, world, local_rank, True, dump_dir=args.dump_outputs)
     second_key = "c4" if args.config == "c3" else "c3"
     second = None
     if not args.no_second:
-        K2 = max(10, min(K, 50 if second_key == "c4" else K))
+        K2 = min(K, 50 if second_key == "c4" else K)
         second = measure(rr, grp, second_key, K2, max(3, min(W, 5 if second_key == "c4" else W)), rank, world, local_rank, False)
     clocks = sampler.stop() if sampler else None
     if rank == 0:
@@ -441,6 +508,8 @@ def run_pf(args):
         g.time_main_kernel(False)
         return dt_, s0, s1
     tt, st0, st1 = flushed(False)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, pf_outputs(g))
     tt_b, _, stb = flushed(True)
     t0 = time.perf_counter()
     for k in range(K):
@@ -508,7 +577,14 @@ def main():
                     help="fastslam workload: 1 = FastSLAM 1.0 (the headline), 2 = FastSLAM 2.0 (fastslam2.rs) on the same configurations")
     ap.add_argument("--particles", type=int, default=1 << 20, help="mcl / pf workloads only")
     ap.add_argument("--threshold", type=float, default=1.0, help="pf workload: resample_threshold (1.0 = resample every step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of the K steps `value` is quoted on computed to DIR/<name>.npy "
+                         "(float64; large arrays as a fixed, seeded sample; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference" and args.workload == "fastslam":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     global NTH_MODE, VARIANT
     NTH_MODE = args.nth
     VARIANT = args.variant
